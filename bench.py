@@ -8,6 +8,7 @@ seeded random weights (no checkpoints offline), bf16 storage / f32 accumulate.
   python bench.py [--gpus N] [--steps K] [--warmup W]            # own arm (CUDA engine, libwkb200.so)
   python bench.py --impl reference [--steps K] [--warmup W]      # CPU restatement of the reference pipeline
   torchrun --nproc-per-node N bench.py --gpus N ...              # one rank per GPU (weak scaling: B windows per GPU)
+  python bench.py ... --dump-outputs DIR                         # also write the last timed step's per-window results to DIR/*.npy
 
 `value`  : device-timed RTFx with the PCM already resident in HBM.
 `e2e`    : the same metric through the public API with HOST buffers: pinned PCM -> (N>1: NCCL scatter) -> GPU ->
@@ -75,7 +76,15 @@ def parse_args():
     ap.add_argument("--chunking", default="vad", choices=["vad", "none"],
                     help="long-form: 'vad' = chunkingStrategy .vad (every stream is cut into independent <= 30 s chunks, WhisperKit.swift:878-911: the "
                          "'chunked to 30 s windows' of BASELINE configs[4]); 'none' = one sequential seek loop per stream")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the per-window decode results of the last device-resident step as DIR/<field>.npy "
+                         "(float32 / float64, at most 64 MB in all) so that two builds can be compared output for output")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "own" or args.longform or args.profile_pass):
+        ap.error("--dump-outputs covers the windowed GPU path only (not --impl reference, --longform or --profile-pass)")
+    return args
 
 
 def eot_profile_lengths(n: int, seed: int = 4321) -> np.ndarray:
@@ -254,7 +263,6 @@ def run_reference_arm(args):
     threads = os.cpu_count() or 1
     metric = "RTFx (audio-sec/s) whisper-large-v3 greedy" if args.variant == "large-v3" else f"RTFx (audio-sec/s) whisper-{args.variant} greedy"
     times = []
-    budget_t0 = time.perf_counter()
     warm = min(args.warmup, 1)  # CPU warm-up = first-touch of the weights; one pass is enough
     for i in range(warm):
         cpu_restatement(args.variant, args.sample_length, args.cpu_windows, threads)
@@ -265,8 +273,6 @@ def run_reference_arm(args):
         log(f"reference step {i}: {dt:.1f} s")
         times.append(dt)
         done += 1
-        if time.perf_counter() - budget_t0 > 360 and done >= 1:
-            break
     total = sum(times)
     value = done * args.cpu_windows * AUDIO_SECONDS_PER_WINDOW / total
     line = {
@@ -287,6 +293,35 @@ def run_reference_arm(args):
 
 
 # ------------------------------------------------------------------------------------------------ own arm
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, res, first_window: int, limit: int = DUMP_LIMIT_BYTES, suffix: str = "") -> None:
+    """Writes what a caller of wk_transcribe_windows_ex receives (one wk_decode_result per window) as out_dir/<field><suffix>.npy,
+    one row per window, plus window_index (the window's number in the seeded PCM sequence).  Integer fields are stored as float64
+    (exact), float fields as float32.  Token slots past a window's n_tokens are not written by the library, so they are stored as
+    -1 (ids) and 0 (log-probs).  When the whole output exceeds `limit` bytes, a fixed seeded sample of windows is written."""
+    a = np.ctypeslib.as_array(res).copy()
+    n = len(a)
+    valid = np.arange(a.dtype["tokens"].shape[0])[None, :] < a["n_tokens"][:, None]
+    fields = {"window_index": np.arange(first_window, first_window + n, dtype=np.float64)}
+    for name in a.dtype.names:
+        v = a[name]
+        if name == "tokens":
+            v = np.where(valid, v, -1)
+        elif name == "token_logprobs":
+            v = np.where(valid, v, 0)
+        fields[name] = v.astype(np.float32 if v.dtype.kind == "f" else np.float64)
+    row_bytes = sum(v.nbytes // n for v in fields.values())
+    if n * row_bytes > limit:
+        keep = np.sort(np.random.default_rng(0).choice(n, limit // row_bytes, replace=False))
+        fields = {k: v[keep] for k, v in fields.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in fields.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), v)
+    log(f"wrote {len(fields)} arrays ({len(fields['window_index'])} of {n} windows) to {out_dir}")
+
+
 def run_own_arm(args):
     import torch
     import whisperkit_b200 as wk
@@ -412,6 +447,8 @@ def run_own_arm(args):
         return
     ms, launches, clocks, _ = timed(step_device, args.steps, max(args.warmup, 3), True)
     log(f"device-resident arm: {ms / args.steps:.1f} ms/step")
+    if args.dump_outputs:   # before the e2e and other-dtype passes reuse `res`
+        dump_outputs(args.dump_outputs, res, rank * W, DUMP_LIMIT_BYTES // world, f"_rank{rank}" if world > 1 else "")
     steps_run = [r.steps for r in res]
     timings = model.last_timings()
     # the e2e region ends when the token IDs are on the host: the library call returns with them, so the wall clock of the calls is the
