@@ -125,6 +125,16 @@ typedef struct wk_decode_opts {
      * word timestamps do not combine with it. */
     int32_t beam_size;            /* <= 1: greedy / temperature sampling (default) */
     float beam_patience;          /* default 1 */
+    /* DecodingOptions.detectLanguage (Configurations.swift:222, default !usePrefillPrompt; 0 here keeps every decode in the given language).
+     * Honoured by decodeWithFallback's entry points (wk_transcribe_windows(_ex), wk_transcribe_windows_sharded, wk_transcribe_streams) for a
+     * multilingual model and language_token < 0: every ladder rung first samples the window's language from the decoder's logits on
+     * [SOT] (TranscribeTask.swift:339-365, TextDecoder.swift:420-539) with the session's language tokens (wk_session_set_language_tokens)
+     * and the rung's temperature, then decodes with it in the prompt's language position (the token after the first SOT, if that token is
+     * a language token; otherwise the detection is only reported).  A prompt that starts with SOT costs no extra decoder pass (the detection
+     * rides on step 0); one that starts with <|startofprev|> costs one.  wk_decode_text(_ex) ignore it (decodeText never detects); with
+     * beam_size > 1 the call fails with WK_ERR_INVALID_ARGUMENT.  Languages come back through wk_session_languages /
+     * wk_transcription_language, wk_decode_result is unchanged. */
+    int32_t detect_language;
 } wk_decode_opts;
 
 /* Per-window DecodingResult (Models.swift:383-439) in flat arrays; tokens = SOT..EOT slice. */
@@ -212,6 +222,17 @@ wk_status wk_decode_text(wk_session* s, const wk_special_tokens* st, const wk_de
  * live when their burst started (an upper bound of the rows that actually streamed K/V), [2] windows admitted to a slot, [3] ladder
  * re-admissions. */
 wk_status wk_session_stats(const wk_session* s, int64_t* out4);
+/* allLanguageTokens of this session (WhisperTokenizerWrapper.allLanguageTokens, Models.swift:1219): the ids detectLanguage chooses from,
+ * and the ids recognised as a language in a decoded window.  n <= 4096, every id inside the vocabulary; n = 0 restores the default: the
+ * ids strictly between start_of_transcript_token and min(translate_token, transcribe_token) of the call's special tokens (the language
+ * block of every Whisper vocabulary: 99 ids, 100 in large-v3).  Per session, so setting it races no other thread. */
+wk_status wk_session_set_language_tokens(wk_session* s, const int32_t* tokens, int32_t n);
+/* The language of the first n windows of the session's last wk_transcribe_windows(_ex) call, as the reference's
+ * `detectedLanguage ?? defaultLanguageCode` (TranscribeTask.swift:341-376): the detected token of the ladder rung whose result was kept
+ * (logprob = the detection step's log-probability, DecodingResult.languageProbs); else the explicit language_token (logprob 0); else the
+ * first language token of the result's tokens (TextDecoder.swift:804-822; logprob = its token_logprobs entry); else english_token (0).
+ * logprobs may be NULL.  After wk_transcribe_windows_sharded every rank holds the languages of its own shard: they are not gathered. */
+wk_status wk_session_languages(const wk_session* s, int64_t n, int32_t* tokens, float* logprobs);
 /* Device logits of the last step, copied to host (debug / parity). */
 wk_status wk_session_last_logits(wk_session* s, float* logits_out);
 
@@ -317,6 +338,10 @@ wk_status wk_transcription_segments(const wk_transcription* t, wk_segment* segs,
 wk_status wk_transcription_tokens(const wk_transcription* t, int32_t* tokens, float* logprobs, int64_t cap);
 int32_t wk_transcription_word_count(const wk_transcription* t);
 wk_status wk_transcription_word(const wk_transcription* t, int32_t i, wk_word* out);   /* .segment indexes wk_transcription_segments */
+/* TranscriptionResult.language of one stream (token, and the log-probability wk_session_languages gives for that window): with detection
+ * on, the last window's detection (detectedLanguage is reassigned every window, TranscribeTask.swift:352); with it off, the first window's
+ * language (:376).  A VAD-chunked stream takes its first chunk's (TranscriptionUtilities.swift:103); a stream with no window, english_token. */
+wk_status wk_transcription_language(const wk_transcription* t, int32_t stream, int32_t* token, float* logprob);
 void wk_transcription_free(wk_transcription* t);
 
 /* ---- word timestamps (SURVEY section 8f row 1) ----
@@ -403,6 +428,9 @@ wk_status wk_tokenizer_special_tokens(const wk_tokenizer* t, wk_special_tokens* 
  * byte inside a decoded word is dropped). */
 int32_t wk_tokenizer_split_to_word_tokens(const wk_tokenizer* t, const int32_t* tokens, int32_t n, char* text, int32_t text_cap, int32_t* counts,
                                           int32_t counts_cap);
+/* WhisperTokenizerWrapper.allLanguageTokens (Models.swift:1219), from the vocabulary: the ids of the added tokens whose content is "<|" + 2
+ * or 3 lowercase ASCII letters + "|>", ascending.  Returns the count, or -(count needed) if cap is short. */
+int32_t wk_tokenizer_language_tokens(const wk_tokenizer* t, int32_t* out, int32_t cap);
 /* Fills `hooks` with this tokenizer's split / decode so wk_transcribe_streams and wk_add_word_timestamps run without host callbacks. */
 wk_status wk_tokenizer_hooks_init(wk_tokenizer* t, wk_tokenizer_hooks* hooks);
 

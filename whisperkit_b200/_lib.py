@@ -63,6 +63,7 @@ class wk_decode_opts(C.Structure):
         ("temperature_fallback_count", C.c_int32), ("temperature_increment_on_fallback", C.c_float),
         ("word_timestamps", C.c_int32),
         ("beam_size", C.c_int32), ("beam_patience", C.c_float),
+        ("detect_language", C.c_int32),
     ]
 
 
@@ -140,6 +141,8 @@ SYMBOLS = [
                              C.POINTER(wk_decode_result)]),
     ("wk_session_last_logits", I32, [P, P]),
     ("wk_session_stats", I32, [P, PI64]),
+    ("wk_session_set_language_tokens", I32, [P, PI32, I32]),
+    ("wk_session_languages", I32, [P, I64, PI32, PF32]),
     ("wk_decode_text_ex", I32, [P, C.POINTER(wk_special_tokens), C.POINTER(wk_batch_opts), C.POINTER(wk_decode_result)]),
     ("wk_transcribe_windows_ex", I32, [P, P, P, I64, I64, PI32, C.POINTER(wk_special_tokens), C.POINTER(wk_batch_opts),
                                        C.POINTER(wk_decode_result)]),
@@ -170,6 +173,7 @@ SYMBOLS = [
     ("wk_transcription_tokens", I32, [P, PI32, PF32, I64]),
     ("wk_transcription_word_count", I32, [P]),
     ("wk_transcription_word", I32, [P, I32, C.POINTER(wk_word)]),
+    ("wk_transcription_language", I32, [P, I32, PI32, PF32]),
     ("wk_transcription_free", None, [P]),
     ("wk_model_set_alignment_heads", I32, [P, PI32, I32]),
     ("wk_session_alignment_weights", I32, [P, I32, I32, P]),
@@ -197,6 +201,7 @@ SYMBOLS = [
     ("wk_tokenizer_set_merges", I32, [P, C.POINTER(C.c_char_p), C.POINTER(C.c_char_p), I32]),
     ("wk_tokenizer_special_tokens", I32, [P, C.POINTER(wk_special_tokens)]),
     ("wk_tokenizer_split_to_word_tokens", I32, [P, PI32, I32, C.POINTER(C.c_char), I32, PI32, I32]),
+    ("wk_tokenizer_language_tokens", I32, [P, PI32, I32]),
     ("wk_tokenizer_hooks_init", I32, [P, C.POINTER(wk_tokenizer_hooks)]),
     ("wk_format_time", I32, [F32, I32, C.c_char_p, C.POINTER(C.c_char), I32]),
     ("wk_write_srt", I32, [PF32, PF32, C.POINTER(C.c_char_p), I32, C.POINTER(C.c_char), I32]),

@@ -91,6 +91,7 @@ class DecodingOptions:
     seed: int = 0
     beamSize: int = 1                 # extension: the reference's BeamSearchTokenSampler is an unimplemented stub (TokenSampler.swift:254-290)
     beamPatience: float = 1.0
+    detectLanguage: Optional[bool] = None   # None = !usePrefillPrompt (Configurations.swift:222)
 
     def to_c(self):
         """Returns (struct, keepalive) - keepalive holds the int arrays the struct points into."""
@@ -132,6 +133,7 @@ class DecodingOptions:
         o.word_timestamps = int(self.wordTimestamps)
         o.beam_size = int(self.beamSize)
         o.beam_patience = float(self.beamPatience)
+        o.detect_language = int(not self.usePrefillPrompt if self.detectLanguage is None else self.detectLanguage)
         return o, keep
 
 
@@ -153,6 +155,9 @@ class DecodingResult:
     currentTokenCount: int = 0
     steps: int = 0
     isFirstTokenLogProbTooLow: bool = False
+    languageToken: Optional[int] = None        # set by WhisperKit.transcribe (wk_session_languages)
+    languageProbs: Dict[object, float] = field(default_factory=dict)   # {language (code, or token id without a tokenizer): log-probability}
+    language: Optional[str] = None             # the code ("en"), when the WhisperKit has a tokenizer
 
     @staticmethod
     def from_c(r: wk_decode_result) -> "DecodingResult":
@@ -423,6 +428,18 @@ class TextDecoder:
         check(self.lib.wk_detect_language(self.handle, C.byref(st), lang, len(allLanguageTokens), float(temperature), tok, lp))
         return list(tok), list(lp)
 
+    def setLanguageTokens(self, tokens: Sequence[int]) -> None:
+        """allLanguageTokens of this session (detectLanguage's choices); [] restores the special tokens' language block."""
+        arr = (C.c_int32 * max(1, len(tokens)))(*[int(t) for t in tokens])
+        check(self.lib.wk_session_set_language_tokens(self.handle, arr, len(tokens)))
+
+    def languages(self, n: int):
+        """[(language token, log-probability)] of the first n windows of the last transcribe call (wk_session_languages)."""
+        tok = (C.c_int32 * max(1, n))()
+        lp = (C.c_float * max(1, n))()
+        check(self.lib.wk_session_languages(self.handle, n, tok, lp))
+        return [(int(tok[i]), float(lp[i])) for i in range(n)]
+
     def alignmentWeights(self, window: int, rows: int = MAX_TOKEN_CONTEXT) -> np.ndarray:
         """DecodingResult.cache.alignmentWeights of one window of the last decodeText(wordTimestamps: true): [rows, 1500] (Float16 values)."""
         out = np.empty((rows, self.model.info.n_audio_ctx), dtype=np.float32)
@@ -561,6 +578,8 @@ class WhisperKit:
         self.featureExtractor = FeatureExtractor(self.model)
         self.audioEncoder = AudioEncoder(self.model)
         self.textDecoder = TextDecoder(self.model, config.maxBatch)
+        if self.tokenizer is not None:   # allLanguageTokens from the tokenizer's vocabulary (Models.swift:1219)
+            self.textDecoder.setLanguageTokens(self.tokenizer.allLanguageTokens)
         info = self.model.info
         if config.specialTokens is not None:
             self.specialTokens = config.specialTokens
@@ -619,10 +638,21 @@ class WhisperKit:
         check(self.model.lib.wk_transcribe_windows_ex(self.model.handle, self.textDecoder.handle, _ptr(a), n, stride, spw, C.byref(st),
                                                       C.byref(bo), res))
         self.textDecoder.batch = min(n, self.config.maxBatch)
+        langs = self.textDecoder.languages(n)
         out = []
         for i, r in enumerate(res):
             if returnErrors and status[i] != 0:
                 out.append(WhisperError(int(status[i]), f"window {i} failed"))
             else:
-                out.append(DecodingResult.from_c(r))
+                d = DecodingResult.from_c(r)
+                d.languageToken, lp = langs[i]
+                d.language = self.languageCode(d.languageToken)
+                d.languageProbs = {d.language if d.language is not None else d.languageToken: lp}
+                out.append(d)
         return out
+
+    def languageCode(self, token: int) -> Optional[str]:
+        """Language token -> code through the tokenizer ("<|de|>" -> "de"); None without a tokenizer."""
+        if self.tokenizer is None:
+            return None
+        return self.tokenizer.decode([int(token)]).removeprefix("<|").removesuffix("|>")

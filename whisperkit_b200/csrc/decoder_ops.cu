@@ -60,6 +60,8 @@ __global__ void decode_slots_init_kernel(DecodeState st, RowParams* __restrict__
         st.steps[b] = 0;
         st.input_ids[b] = 0;
         st.error[b] = 0;
+        st.lang_tok[b] = -1;
+        st.lang_lp[b] = 0.f;
         if (bs.beam > 1) {
             bs.sum_lp[b] = 0.f;
             if (b % bs.beam == 0) bs.n_fin[b / bs.beam] = 0;
@@ -83,7 +85,7 @@ wk_status decode_slots_init(DecodeState st, RowParams* rp_dev, const int32_t* sl
 template <typename T>
 __global__ void __launch_bounds__(256)
 decoder_embed_ln_kernel(const T* __restrict__ emb, const float* __restrict__ pos_emb, const float* __restrict__ gamma,
-                        const float* __restrict__ beta, DecodeState st, int vocab, int ts_begin, float* __restrict__ x,
+                        const float* __restrict__ beta, DecodeState st, int vocab, int ts_begin, int sot, float* __restrict__ x,
                         T* __restrict__ xn, int d, const int32_t* __restrict__ explicit_pos) {
     __shared__ float scratch[32];
     const int b = blockIdx.x, tid = threadIdx.x;
@@ -100,7 +102,9 @@ decoder_embed_ln_kernel(const T* __restrict__ emb, const float* __restrict__ pos
         pos = step;
         tok = st.next_token[b];
         bool overwrite = false;
-        if (step < prompt_len) {
+        if (step == 0 && (st.rp[b].lang_flags & kLangPreStep) && st.lang_tok[b] < 0) {
+            tok = sot;                   // language-detection pre-step: SOT at position 0 (the prompt's own step 0 overwrites its K/V row)
+        } else if (step < prompt_len) {
             const int cur = st.tokens[b * kMaxCtx + step];
             const bool is_ts = cur >= ts_begin, pred_ts = tok >= ts_begin;
             if (!(step == prompt_len - 1 && is_ts && pred_ts)) tok = cur;
@@ -141,12 +145,12 @@ decoder_embed_ln_kernel(const T* __restrict__ emb, const float* __restrict__ pos
 }
 
 wk_status decoder_embed_ln(const void* emb16, const float* pos, const float* gamma, const float* beta, DecodeState st, int vocab,
-                           int ts_begin, float* x, void* xn, int B, int d, int dtype, const int32_t* explicit_pos, cudaStream_t stream) {
+                           int ts_begin, int sot, float* x, void* xn, int B, int d, int dtype, const int32_t* explicit_pos, cudaStream_t stream) {
     if (d > 2048) { set_error("decoder_embed_ln: d_model %d > 2048", d); return WK_ERR_INVALID_ARGUMENT; }
     if (dtype == WK_DTYPE_F16)
-        launch_k(decoder_embed_ln_kernel<__half>, dim3(B), dim3(256), 0, stream, 1, (const __half*)emb16, pos, gamma, beta, st, vocab, ts_begin, x, (__half*)xn, d, explicit_pos);
+        launch_k(decoder_embed_ln_kernel<__half>, dim3(B), dim3(256), 0, stream, 1, (const __half*)emb16, pos, gamma, beta, st, vocab, ts_begin, sot, x, (__half*)xn, d, explicit_pos);
     else
-        launch_k(decoder_embed_ln_kernel<__nv_bfloat16>, dim3(B), dim3(256), 0, stream, 1, (const __nv_bfloat16*)emb16, pos, gamma, beta, st, vocab, ts_begin, x, (__nv_bfloat16*)xn, d, explicit_pos);
+        launch_k(decoder_embed_ln_kernel<__nv_bfloat16>, dim3(B), dim3(256), 0, stream, 1, (const __nv_bfloat16*)emb16, pos, gamma, beta, st, vocab, ts_begin, sot, x, (__nv_bfloat16*)xn, d, explicit_pos);
     count_launch();
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) { set_error("decoder_embed_ln launch: %s", cudaGetErrorString(e)); return WK_ERR_CUDA; }
@@ -592,8 +596,9 @@ __global__ void decoder_align_mean_kernel(const float* __restrict__ scratch, int
     // launched after the sampler advanced the row's step: steps[b] = tokenIndex + 1 = the row of this step's slice; a window whose
     // segment just completed (or completed earlier) gets no row - the reference breaks out of its loop before updateAlignmentWeights
     // (TextDecoder.swift:668-674,709-717)
+    // (row 0 is never a step's row: steps[b] is still 0 only after a language-detection pre-step, which has no alignment row)
     const int row = steps[b];
-    if (t >= Tlen || row >= max_rows || done[b]) return;
+    if (t >= Tlen || row < 1 || row >= max_rows || done[b]) return;
     float a = 0.f;
     for (int s = 0; s < n_slots; ++s) a += scratch[((long long)s * B + b) * Tlen + t];   // fixed order: deterministic
     out[((long long)b * max_rows + row) * Tlen + t] = __float2half(a / (float)n_slots);
@@ -675,11 +680,18 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
     const int32_t* toks = loop_mode ? st.tokens + b * kMaxCtx : tokens_in + (long long)b * ld_tokens;
     const int n_tok = loop_mode ? st.n_tokens[b] : n_tokens_in[b];
     const wk_special_tokens& S = p.st;
-
+    // DecodingOptions.detectLanguage (TranscribeTask.swift:339-365, TextDecoder.swift:420-539): a detecting row's first pass runs SOT at
+    // position 0, so its logits are detectLanguage's.  Pass 0 samples the language from them (LanguageLogitsFilter, then the rung's
+    // sampler; no other filter); pass 1 is the ordinary step.  A pre-step (prompt not starting with SOT) runs pass 0 only.  The branch is
+    // per row: rows that do not detect run pass 1 alone.
+    const bool detect = loop_mode && R.lang_flags != 0 && st.steps[b] == 0 && st.lang_tok[b] < 0;
+    const bool prestep = detect && (R.lang_flags & kLangPreStep) != 0;
+    for (int pass = detect ? 0 : 1; pass < (prestep ? 1 : 2); ++pass) {
+    const bool lang_pass = pass == 0;
     if (tid == 0) {
         // ---- TimestampRulesFilter rule state (LogitsFilter.swift:72-109)
         int active = 0, loA = 0, hiA = 0, loB = 0, hiB = 0;
-        if (R.sample_begin_ts >= 0) {
+        if (!lang_pass && R.sample_begin_ts >= 0) {
             int sb = -1;
             if (p.is_multilingual) {
                 const int lim = n_tok < 3 ? n_tok : 3;
@@ -709,8 +721,8 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
             }
         }
         sflag[0] = active; sflag[1] = loA; sflag[2] = hiA; sflag[3] = loB; sflag[4] = hiB;
-        sflag[5] = (R.sample_begin_blank >= 0 && n_tok == R.sample_begin_blank) ? 1 : 0;   // SuppressBlankFilter
-        sflag[6] = (p.language_tokens != nullptr && n_tok >= p.language_sample_begin) ? 1 : 0;  // LanguageLogitsFilter
+        sflag[5] = (!lang_pass && R.sample_begin_blank >= 0 && n_tok == R.sample_begin_blank) ? 1 : 0;   // SuppressBlankFilter
+        sflag[6] = (lang_pass || (!loop_mode && p.language_tokens != nullptr && n_tok >= p.language_sample_begin)) ? 1 : 0;  // LanguageLogitsFilter
     }
     __syncthreads();
     const int ts_active = sflag[0], loA = sflag[1], hiA = sflag[2], loB = sflag[3], hiB = sflag[4];
@@ -743,7 +755,7 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
         }
         __syncthreads();
     }
-    for (int j = tid; j < R.n_suppress; j += kSamplerThreads) {   // SuppressTokensFilter
+    for (int j = tid; j < (lang_pass ? 0 : R.n_suppress); j += kSamplerThreads) {   // SuppressTokensFilter
         const int t = p.suppress[R.suppress_off + j];
         if (t >= 0 && t < V) srow[t] = -INFINITY;
     }
@@ -814,7 +826,7 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
         }
         return best;   // identical in every thread
     };
-    if (loop_mode && p.beam.beam > 1) {
+    if (loop_mode && !lang_pass && p.beam.beam > 1) {
         // beam search: rank the row's (beam + 1) best tokens of the filtered log-softmax, best first (whisper BeamSearchDecoder.update step 1);
         // the per-window merge and every state update happen in beam_update_kernel
         const int k = p.beam.beam + 1;
@@ -838,7 +850,8 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
     } else {
         // GreedyTokenSampler with temperature (TokenSampler.swift:57-73 / :140-180): logits / T, softmax over the whole
         // (filtered) vocabulary, top-k, multinomial draw inside the top-k mass, logprob = log softmax prob of the draw.
-        // The reference draws with Float.random (non-deterministic); here the draw is Philox(seed, row, step).
+        // The reference draws with Float.random (non-deterministic); here the draw is Philox(seed, row, step).  The language draw uses
+        // subsequence 2^32 + row, which no token draw of any row reaches.
         const float inv_t = 1.f / R.temperature;
         const float zmax = (ts_wins ? mts : mall) * inv_t;
         float z = 0.f;
@@ -861,7 +874,8 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
         float mass = 0.f;
         for (int j = 0; j < kk; ++j) mass += topv[j];
         curandStatePhilox4_32_10_t rng;
-        curand_init(R.seed, (unsigned long long)b, (unsigned long long)(loop_mode ? st.steps[b] : n_tok), &rng);
+        if (lang_pass) curand_init(R.seed, (1ull << 32) + (unsigned long long)b, 0ull, &rng);
+        else curand_init(R.seed, (unsigned long long)b, (unsigned long long)(loop_mode ? st.steps[b] : n_tok), &rng);
         const float u = 1.f - curand_uniform(&rng);   // [0, 1)
         const float rnd = u * mass;
         float acc = 0.f;
@@ -880,6 +894,15 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
         // a row with no finite logit (every token masked, or a NaN from upstream) has no argmax: end the window there and flag it instead
         // of feeding an out-of-range id to the next embedding lookup (the host reports WhisperError.decodingLogitsFailed for the window)
         const bool bad = tok < 0 || tok >= V;
+        sflag[7] = lang_pass && bad;
+        if (lang_pass) {
+            // the detected language; the embed kernel forces it at the prompt's language position
+            if (bad) { st.error[b] = 1; st.done[b] = 1; }
+            else {
+                st.lang_tok[b] = tok; st.lang_lp[b] = lp;
+                if (R.lang_slot >= 0) st.tokens[b * kMaxCtx + R.lang_slot] = tok;
+            }
+        } else {
         if (bad) { tok = S.end_token; lp = -INFINITY; }
         if (token_out) token_out[b] = bad ? -1 : tok;
         if (logprob_out) logprob_out[b] = lp;
@@ -903,6 +926,12 @@ sampler_kernel(const float* __restrict__ logits, long long ld_logits, SamplerPar
                 if (step + 1 >= R.max_steps) st.done[b] = 1;   // loop bound min(sampleLength, 223) reached (TextDecoder.swift:566)
             }
         }
+        }
+    }
+    if (lang_pass) {   // (uniform over the CTA) pass 1 restages srow; a row without a finite language logit ends here
+        __syncthreads();
+        if (sflag[7]) return;
+    }
     }
 }
 

@@ -103,8 +103,14 @@ struct RowParams {
     int32_t has_first_thr; float first_thr;
     uint64_t seed;
     int32_t suppress_off, n_suppress;   // slice of the session's suppress-token pool
-    int32_t pad_[2];
+    // DecodingOptions.detectLanguage (TranscribeTask.swift:339-365): the row samples its language from the logits of SOT at position 0
+    // (LanguageLogitsFilter over SamplerParams.language_tokens, then the rung's sampler) before its decode goes on
+    int32_t lang_slot;           // prompt position the detected language is written to (the token after the first SOT), -1 = none
+    int32_t lang_flags;          // kLangDetect | kLangPreStep
 };
+// kLangDetect: the row detects at step 0 (its prompt starts with SOT, so step 0 already runs SOT at position 0).
+// kLangPreStep: the prompt starts elsewhere (<|startofprev|>): one extra pass feeds SOT at position 0, detects, and leaves steps at 0.
+constexpr int32_t kLangDetect = 1, kLangPreStep = 2;
 
 struct DecodeState {
     // all device pointers; one entry per decode row (slot).  A slot with done != 0 is skipped by every kernel of the step.
@@ -118,6 +124,8 @@ struct DecodeState {
     int32_t* input_ids;   // [Bmax] token fed at this step (written by embed)
     int32_t* error;       // [Bmax] 1 = the sampler saw no finite logit (WhisperError.decodingLogitsFailed)
     const RowParams* rp;  // [Bmax]
+    int32_t* lang_tok;    // [Bmax] detected language token, -1 = not detected (yet)
+    float* lang_lp;       // [Bmax] its log-probability under the language filter
 };
 
 // Beam search (SURVEY 8f row 2; semantics restated from openai/whisper BeamSearchDecoder in oracle/beam_ref.py - the reference's
@@ -141,6 +149,8 @@ struct SamplerParams {
     int is_multilingual;
     int loop_mode;           // 1: decode loop (per-row options from DecodeState.rp); 0: stateless (wk_filter_sample / detectLanguage)
     const int32_t* suppress; // loop mode: the pool RowParams.suppress_off indexes; stateless: the list itself
+    // stateless: LanguageLogitsFilter(sampleBegin = language_sample_begin); loop mode: the session's allLanguageTokens, read only at the
+    // detection step of rows with RowParams.lang_flags set
     const int32_t* language_tokens; int n_language_tokens; int language_sample_begin;
     int max_ctx;             // 224
     BeamState beam;          // loop mode with beam.beam > 1: the kernel only ranks candidates; beam_update() does the bookkeeping
@@ -149,9 +159,9 @@ struct SamplerParams {
     float temperature; int top_k; uint64_t seed;
 };
 
-// pos: explicit per-row positions (wk_decode_step) or nullptr = DecodeState.steps
+// pos: explicit per-row positions (wk_decode_step) or nullptr = DecodeState.steps.  sot: the token a language-detection pre-step feeds
 wk_status decoder_embed_ln(const void* emb16, const float* pos, const float* gamma, const float* beta, DecodeState st, int vocab,
-                           int ts_begin, float* x, void* xn, int B, int d, int dtype, const int32_t* explicit_pos, cudaStream_t stream);
+                           int ts_begin, int sot, float* x, void* xn, int B, int d, int dtype, const int32_t* explicit_pos, cudaStream_t stream);
 // x[b,:] += bias + sum_s partial[s][b][:]; xn = LN(x) (16-bit).  partial layout [S][Bp][d]
 wk_status decoder_reduce_resid_ln(const float* partial, int splits, int Bp, const float* bias, const float* gamma,
                                   const float* beta, float* x, void* xn, int B, int d, int dtype, cudaStream_t stream);

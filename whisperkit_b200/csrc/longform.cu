@@ -239,6 +239,8 @@ struct wk_transcription {
     std::vector<int32_t> tokens;
     std::vector<float> logprobs;
     int windows = 0;
+    std::vector<int32_t> lang_tok;   // per stream: TranscriptionResult.language
+    std::vector<float> lang_lp;
 };
 
 namespace {
@@ -253,6 +255,8 @@ struct Unit {                 // one independently advancing cursor: a stream, o
     bool done = false;
     std::vector<wk_segment> segs;
     std::vector<OutWord> words;   // word timings; .segment indexes `segs`
+    int windows = 0;
+    int32_t lang_tok = -1; float lang_lp = 0.f;   // the unit's detectedLanguage (first or last window's, see wk_transcription_language)
 };
 }  // namespace
 
@@ -369,6 +373,10 @@ wk_status wk_transcribe_streams(wk_model* m, wk_session* s, const float* const* 
     float* batch = hs.pcm;
     std::vector<int32_t> valid(round_cap);
     std::vector<wk_decode_result> res(round_cap);
+    std::vector<int32_t> win_lang(round_cap);
+    std::vector<float> win_lang_lp(round_cap);
+    // detectedLanguage is reassigned every window when the task detects (TranscribeTask.swift:352), set once otherwise (:376)
+    const bool detecting = info.is_multilingual && o->detect_language && o->language_token < 0;
     std::vector<int> active;
     std::vector<std::vector<int32_t>> unit_tokens(units.size());
     std::vector<std::vector<float>> unit_lps(units.size());
@@ -391,6 +399,12 @@ wk_status wk_transcribe_streams(wk_model* m, wk_session* s, const float* const* 
         rc = wk_transcribe_windows(m, s, batch, (int64_t)active.size(), kWindow, valid.data(), st, o, prompt, n_prompt, res.data());
         if (rc != WK_OK) { delete T; return rc; }
         T->windows += (int)active.size();
+        rc = wk_session_languages(s, (int64_t)active.size(), win_lang.data(), win_lang_lp.data());
+        if (rc != WK_OK) { delete T; return rc; }
+        for (size_t k = 0; k < active.size(); ++k) {
+            Unit& u = units[active[k]];
+            if (u.windows++ == 0 || detecting) { u.lang_tok = win_lang[k]; u.lang_lp = win_lang_lp[k]; }
+        }
         const int cols = info.n_audio_ctx;
         if (o->word_timestamps) {   // every window's alignment rows back in one burst (Float16, as the reference's alignmentWeights)
             for (size_t k = 0; k < active.size(); ++k) {
@@ -474,6 +488,16 @@ wk_status wk_transcribe_streams(wk_model* m, wk_session* s, const float* const* 
     }
     // flatten: streams in order, units (chunks) in order, chunk offsets applied (updateSegmentTimings, AudioChunker.swift:14-39)
     std::vector<int> next_id(n_streams, 0);
+    // a stream's language is its first unit's: a plain stream has one, a VAD-chunked stream takes its first chunk's
+    // (TranscriptionUtilities.swift:103); a stream without a window reports English
+    T->lang_tok.assign(n_streams, st->english_token);
+    T->lang_lp.assign(n_streams, 0.f);
+    std::vector<uint8_t> lang_set(n_streams, 0);
+    for (const Unit& u : units)
+        if (!lang_set[u.stream]) {
+            lang_set[u.stream] = 1;
+            if (u.windows > 0) { T->lang_tok[u.stream] = u.lang_tok; T->lang_lp[u.stream] = u.lang_lp; }
+        }
     for (size_t i = 0; i < units.size(); ++i) {
         Unit& u = units[i];
         const float seek_time = (float)u.offset / (float)kSampleRate;
@@ -518,6 +542,12 @@ wk_status wk_transcription_word(const wk_transcription* t, int32_t i, wk_word* o
     const OutWord& w = t->words[i];
     out->word = w.word.c_str(); out->tokens = w.tokens.data(); out->n_tokens = (int32_t)w.tokens.size();
     out->start = w.start; out->end = w.end; out->probability = w.probability; out->segment = w.segment;
+    return WK_OK;
+}
+wk_status wk_transcription_language(const wk_transcription* t, int32_t stream, int32_t* token, float* logprob) {
+    if (!t || !token || stream < 0 || stream >= (int32_t)t->lang_tok.size()) { set_error("wk_transcription_language: stream out of range"); return WK_ERR_INVALID_ARGUMENT; }
+    *token = t->lang_tok[stream];
+    if (logprob) *logprob = t->lang_lp[stream];
     return WK_OK;
 }
 void wk_transcription_free(wk_transcription* t) { delete t; }

@@ -67,6 +67,12 @@ struct wk_session {
     int graph_beam = 1;
     std::vector<int> slot_window, slot_try;
     int64_t stats[4] = {0, 0, 0, 0};   // of the last batched call: step launches, sum of live rows over them, admissions, ladder re-admissions
+    // language detection: the session's allLanguageTokens (empty = the special tokens' language block), the list length baked into the
+    // step graphs, the pinned readback of the rows' detections and the language of every window of the last wk_transcribe_windows(_ex)
+    std::vector<int32_t> lang_list;
+    int graph_lang_n = 0, loop_lang_n = 0;
+    int32_t* h_lang_tok = nullptr; float* h_lang_lp = nullptr;
+    std::vector<int32_t> win_lang_tok; std::vector<float> win_lang_lp;
 };
 
 namespace wk {
@@ -94,7 +100,7 @@ static wk_status dec_gemm(wk_session* s, const void* w, int N, int K, const void
 static bool use_fused(const wk_session* s) { return s->knob_fused && s->m->live_sessions.load(std::memory_order_relaxed) == 1; }
 
 // one decoder forward for every row of the step.  explicit_pos == nullptr: loop mode (token / position from DecodeState, ended rows skipped)
-static wk_status decoder_forward(wk_session* s, int ts_begin, const int32_t* explicit_pos, bool fused, bool check_done = true) {
+static wk_status decoder_forward(wk_session* s, int ts_begin, int sot, const int32_t* explicit_pos, bool fused, bool check_done = true) {
     wk_model* m = s->m;
     const wk_model_config& c = m->cfg;
     const int d = c.d_model, H = c.n_heads, dt = c.dtype, B = s->batch, Bp = s->bp, T = c.n_audio_ctx;
@@ -108,7 +114,7 @@ static wk_status decoder_forward(wk_session* s, int ts_begin, const int32_t* exp
     const bool beam_rows = !explicit_pos && s->bs.beam > 1;   // rows are beams: cache ancestry + one cross K/V block per `beam` rows
     const int n_layers = c.dec_layers;
     int sp = 1;
-    WK_CHECK(decoder_embed_ln(m->emb, m->dec_pos, m->dec[0].ln1.g, m->dec[0].ln1.b, s->st, c.vocab, ts_begin, s->x, s->xn, B, d, dt, explicit_pos, st));
+    WK_CHECK(decoder_embed_ln(m->emb, m->dec_pos, m->dec[0].ln1.g, m->dec[0].ln1.b, s->st, c.vocab, ts_begin, sot, s->x, s->xn, B, d, dt, explicit_pos, st));
     auto self_attn = [&](int li, const DecLayer& l) {
         return decoder_self_attention(s->partial, sp, Bp, l.bq, l.bv, (char*)s->self_k + li * self_layer, (char*)s->self_v + li * self_layer, pos, done,
                                       s->attn, B, H, kKvMaxLen, dt, st, beam_rows ? s->bs.anc : nullptr);
@@ -207,6 +213,7 @@ static SamplerParams loop_sampler_params(wk_session* s, const wk_special_tokens*
     p.suppress = s->suppress_dev;
     p.max_ctx = kKvMaxLen;
     p.beam = s->bs;
+    p.language_tokens = s->lang_dev; p.n_language_tokens = s->loop_lang_n;
     return p;
 }
 
@@ -297,7 +304,7 @@ static wk_status build_prompt(const wk_model* m, const wk_special_tokens* st, co
 // ---------------------------------------------------------------------------------------------- the step and its graph
 static wk_status enqueue_step(wk_session* s, const wk_special_tokens* st, bool fused, bool check_done) {
     wk_model* m = s->m;
-    WK_CHECK(decoder_forward(s, st->time_token_begin, nullptr, fused, check_done));
+    WK_CHECK(decoder_forward(s, st->time_token_begin, st->start_of_transcript_token, nullptr, fused, check_done));
     WK_CHECK(sampler_filter_sample(s->logits, m->cfg.vocab, loop_sampler_params(s, st), s->st, nullptr, 0, nullptr, nullptr, nullptr, nullptr, s->batch, s->stream));
     if (s->bs.beam > 1) WK_CHECK(beam_update(s->st, s->bs, *st, kKvMaxLen, s->batch / s->bs.beam, s->stream));
     if (s->align_on)
@@ -319,11 +326,12 @@ static wk_status run_steps(wk_session* s, const wk_special_tokens* st, int n, bo
     if (done >= n) return WK_OK;
     const int beam_key = std::max(1, s->bs.beam) * 16 + s->bs.max_candidates;
     const bool stale = s->graph_batch != s->batch || s->graph_align != s->align_on || s->graph_fused != fused || s->graph_beam != beam_key ||
-                       memcmp(&s->graph_st, st, sizeof(*st)) != 0;
+                       s->graph_lang_n != s->loop_lang_n || memcmp(&s->graph_st, st, sizeof(*st)) != 0;
     if (stale) {
         if (s->graph_exec) { cudaGraphExecDestroy(s->graph_exec); s->graph_exec = nullptr; }
         if (s->graph_exec_live) { cudaGraphExecDestroy(s->graph_exec_live); s->graph_exec_live = nullptr; }
         s->graph_batch = s->batch; s->graph_align = s->align_on; s->graph_fused = fused; s->graph_st = *st; s->graph_beam = beam_key;
+        s->graph_lang_n = s->loop_lang_n;
     }
     cudaGraphExec_t& exec = check_done ? s->graph_exec : s->graph_exec_live;
     if (!exec) {
@@ -413,6 +421,16 @@ static wk_status ensure_beam(wk_session* s) {
     return WK_OK;
 }
 
+// allLanguageTokens of a call (Models.swift:1219): the session's list, else the ids strictly between <|startoftranscript|> and
+// min(<|translate|>, <|transcribe|>) - the language block of every Whisper vocabulary (99 ids, 100 in large-v3)
+static std::vector<int32_t> language_list(const wk_session* s, const wk_special_tokens* st) {
+    if (!s->lang_list.empty()) return s->lang_list;
+    std::vector<int32_t> v;
+    const int hi = std::min(st->translate_token, st->transcribe_token);
+    for (int t = std::max(st->start_of_transcript_token + 1, 0); t < hi && t < s->m->cfg.vocab; ++t) v.push_back(t);
+    return v;
+}
+
 static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
     wk_model* m = s->m;
     const wk_model_config& c = m->cfg;
@@ -439,6 +457,17 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
         for (int i = 0; i < bo->n_opts; ++i)
             if (bo->opts[i].word_timestamps) { set_error("wordTimestamps with beam search is not supported"); return WK_ERR_INVALID_ARGUMENT; }
         WK_CHECK(ensure_beam(s));
+    }
+    // detectLanguage (TranscribeTask.swift:339-365) runs in decodeWithFallback only (the entry points with the ladder), for a multilingual
+    // model and a window without an explicit language
+    const std::vector<int32_t> langs = language_list(s, st);
+    auto detects = [&](const wk_decode_opts& o) { return a.ladder && c.vocab != 51864 && o.detect_language != 0 && o.language_token < 0; };
+    auto is_language = [&](int32_t t) { return std::find(langs.begin(), langs.end(), t) != langs.end(); };
+    bool any_detect = false;
+    for (int i = 0; i < bo->n_opts; ++i) any_detect |= detects(bo->opts[i]);
+    if (any_detect && beam > 1) { set_error("detectLanguage with beam search is not supported"); return WK_ERR_INVALID_ARGUMENT; }
+    if (any_detect && (langs.empty() || langs.size() > 4096)) {
+        set_error("detectLanguage: %zu language tokens (the list must hold 1 .. 4096 ids)", langs.size()); return WK_ERR_INVALID_ARGUMENT;
     }
     s->bs.beam = beam; s->bs.max_candidates = max_cand;
     const int S = s->max_batch / beam;     // decode slots (windows in flight)
@@ -501,6 +530,10 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
         if (s->graph_exec_live) { cudaGraphExecDestroy(s->graph_exec_live); s->graph_exec_live = nullptr; }
     }
     if (!sup_pool.empty()) WK_CUDA_CHECK(cudaMemcpyAsync(s->suppress_dev, sup_pool.data(), sup_pool.size() * 4, cudaMemcpyHostToDevice, s->stream));
+    if (any_detect) {   // (wk_detect_language shares the buffer: the list goes up again with every call that detects)
+        WK_CUDA_CHECK(cudaMemcpyAsync(s->lang_dev, langs.data(), langs.size() * 4, cudaMemcpyHostToDevice, s->stream));
+        s->loop_lang_n = (int)langs.size();
+    }
     WK_CUDA_CHECK(cudaStreamSynchronize(s->stream));   // sup_pool is pageable: the copy must land before it goes out of scope paths below reuse it
     s->align_on = any_words;
     if (any_words) WK_CHECK(ensure_align(s, n));
@@ -541,6 +574,13 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
         R.has_first_thr = o.has_first_token_logprob_threshold; R.first_thr = o.first_token_logprob_threshold;
         R.seed = o.seed + (uint64_t)rung;
         R.suppress_off = sup_off[oi]; R.n_suppress = sup_n[oi];
+        // the language slot: the position after the first SOT, when it holds a language token; without one the detection only reports
+        R.lang_slot = -1; R.lang_flags = 0;
+        if (detects(o)) {
+            R.lang_flags = p[0] == st->start_of_transcript_token ? kLangDetect : kLangPreStep;
+            for (int i = 0; i < np; ++i)
+                if (p[i] == st->start_of_transcript_token) { if (i + 1 < np && is_language(p[i + 1])) R.lang_slot = i + 1; break; }
+        }
         if (n_adm == 0) cudaEventSynchronize(s->ev_stage);   // the previous round's copies out of the pinned staging have landed
         for (int j = 0; j < beam; ++j) {                     // beam search: `beam` identical rows start the window
             s->h_adm_slots[n_adm] = slot * beam + j;
@@ -629,6 +669,21 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
         return gemm_tcgen05(g, m->num_sms, s->stream);
     };
 
+    // TranscriptionResult.language of every window: detectedLanguage ?? defaultLanguageCode (TranscribeTask.swift:341-376) - the kept rung's
+    // detection, else the explicit language, else the first language token of the result (TextDecoder.swift:804-822), else English
+    if (a.ladder) { s->win_lang_tok.assign((size_t)n, st->english_token); s->win_lang_lp.assign((size_t)n, 0.f); }
+    auto record_language = [&](int64_t w, const wk_decode_result& r, int r0) {
+        if (!a.ladder) return;
+        const wk_decode_opts& o = opts_of(bo, w);
+        int32_t tok = st->english_token; float lp = 0.f;
+        if (detects(o)) { tok = s->h_lang_tok[r0]; lp = s->h_lang_lp[r0]; }
+        else if (o.language_token >= 0) tok = o.language_token;
+        else
+            for (int i = 0; i < r.n_tokens; ++i)
+                if (is_language(r.tokens[i])) { tok = r.tokens[i]; lp = r.token_logprobs[i]; break; }
+        s->win_lang_tok[(size_t)w] = tok; s->win_lang_lp[(size_t)w] = lp;
+    };
+
     int64_t finished = 0;
     for (int64_t w = 0; w < n; ++w) if (status[w] != WK_OK) ++finished;
     memset(s->stats, 0, sizeof(s->stats));
@@ -692,6 +747,10 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
         WK_CUDA_CHECK(cudaMemcpyAsync(s->h_error, s->st.error, rows * 4, cudaMemcpyDeviceToHost, s->stream));
         WK_CUDA_CHECK(cudaMemcpyAsync(s->h_tokens, s->st.tokens, (size_t)rows * kKvMaxLen * 4, cudaMemcpyDeviceToHost, s->stream));
         WK_CUDA_CHECK(cudaMemcpyAsync(s->h_logprobs, s->st.logprobs, (size_t)rows * kKvMaxLen * 4, cudaMemcpyDeviceToHost, s->stream));
+        if (any_detect) {
+            WK_CUDA_CHECK(cudaMemcpyAsync(s->h_lang_tok, s->st.lang_tok, rows * 4, cudaMemcpyDeviceToHost, s->stream));
+            WK_CUDA_CHECK(cudaMemcpyAsync(s->h_lang_lp, s->st.lang_lp, rows * 4, cudaMemcpyDeviceToHost, s->stream));
+        }
         if (beam > 1) {
             WK_CUDA_CHECK(cudaMemcpyAsync(s->h_sum_lp, s->bs.sum_lp, rows * 4, cudaMemcpyDeviceToHost, s->stream));
             WK_CUDA_CHECK(cudaMemcpyAsync(s->h_n_fin, s->bs.n_fin, Brun * 4, cudaMemcpyDeviceToHost, s->stream));
@@ -779,6 +838,7 @@ static wk_status transcribe_core(wk_session* s, const CoreArgs& a) {
                 continue;
             } else {
                 a.results[w] = r;
+                record_language(w, r, r0);
             }
             if (s->align_on && status[w] == WK_OK)
                 WK_CUDA_CHECK(cudaMemcpyAsync((char*)s->align_store + (size_t)w * kKvMaxLen * T * 2, (char*)s->align_w + (size_t)q * kKvMaxLen * T * 2,
@@ -850,6 +910,8 @@ wk_status wk_session_create(wk_model* m, int32_t max_batch, wk_session** out) {
     WK_CHECK(dmalloc(&s->st.steps, S));
     WK_CHECK(dmalloc(&s->st.input_ids, S));
     WK_CHECK(dmalloc(&s->st.error, S));
+    WK_CHECK(dmalloc(&s->st.lang_tok, S));
+    WK_CHECK(dmalloc(&s->st.lang_lp, S));
     WK_CHECK(dmalloc(&s->rp_dev, S));
     s->st.rp = s->rp_dev;
     WK_CHECK(dmalloc(&s->pos_dev, S));
@@ -876,6 +938,8 @@ wk_status wk_session_create(wk_model* m, int32_t max_batch, wk_session** out) {
     WK_CHECK(pinned((void**)&s->h_first_low, (size_t)S * 4));
     WK_CHECK(pinned((void**)&s->h_steps, (size_t)S * 4));
     WK_CHECK(pinned((void**)&s->h_error, (size_t)S * 4));
+    WK_CHECK(pinned((void**)&s->h_lang_tok, (size_t)S * 4));
+    WK_CHECK(pinned((void**)&s->h_lang_lp, (size_t)S * 4));
     WK_CUDA_CHECK(cudaEventCreateWithFlags(&s->ev_enc, cudaEventDisableTiming));
     WK_CUDA_CHECK(cudaEventCreateWithFlags(&s->ev_adm, cudaEventDisableTiming));
     WK_CUDA_CHECK(cudaEventCreateWithFlags(&s->ev_stage, cudaEventDisableTiming));
@@ -901,9 +965,10 @@ void wk_session_free(wk_session* s) {
     void* ptrs[] = {s->cross_kv, s->self_k, s->self_v, s->partial, s->x, s->xn, s->attn, s->ffn, s->logits, s->st.tokens, s->st.n_tokens,
                     s->st.logprobs, s->st.next_token, s->st.done, s->st.first_low, s->st.steps, s->st.input_ids, s->st.error, s->rp_dev,
                     s->pos_dev, s->lang_dev, s->suppress_dev, s->d_adm_slots, s->d_adm_prompts, s->d_adm_rp, s->align_scratch, s->align_w,
-                    s->align_store, s->chain_counters};
+                    s->align_store, s->chain_counters, s->st.lang_tok, s->st.lang_lp};
     for (void* p : ptrs) if (p) cudaFree(p);
-    void* hptrs[] = {s->h_adm_slots, s->h_adm_prompts, s->h_adm_rp, s->h_tokens, s->h_logprobs, s->h_n_tokens, s->h_done, s->h_first_low, s->h_steps, s->h_error};
+    void* hptrs[] = {s->h_adm_slots, s->h_adm_prompts, s->h_adm_rp, s->h_tokens, s->h_logprobs, s->h_n_tokens, s->h_done, s->h_first_low, s->h_steps, s->h_error,
+                     s->h_lang_tok, s->h_lang_lp};
     for (void* p : hptrs) if (p) cudaFreeHost(p);
     enc_ws_free(&s->ws);
     cudaEventDestroy(s->ev_enc); cudaEventDestroy(s->ev_adm); cudaEventDestroy(s->ev_stage);
@@ -969,7 +1034,7 @@ wk_status wk_decode_step(wk_session* s, const int32_t* input_ids, const int32_t*
     }
     WK_CUDA_CHECK(cudaMemcpyAsync(s->st.input_ids, input_ids, s->batch * 4, cudaMemcpyHostToDevice, s->stream));
     WK_CUDA_CHECK(cudaMemcpyAsync(s->pos_dev, cache_length, s->batch * 4, cudaMemcpyHostToDevice, s->stream));
-    WK_CHECK(decoder_forward(s, 0, s->pos_dev, use_fused(s)));
+    WK_CHECK(decoder_forward(s, 0, 0, s->pos_dev, use_fused(s)));
     if (logits_out)
         WK_CUDA_CHECK(cudaMemcpyAsync(logits_out, s->logits, (size_t)s->batch * m->cfg.vocab * 4, cudaMemcpyDeviceToHost, s->stream));
     cudaError_t e = cudaStreamSynchronize(s->stream);
@@ -1000,7 +1065,7 @@ wk_status wk_detect_language(wk_session* s, const wk_special_tokens* st, const i
     std::vector<int32_t> ids(B, st->start_of_transcript_token), zeros(B, 0), ones(B, 1);
     WK_CUDA_CHECK(cudaMemcpyAsync(s->st.input_ids, ids.data(), B * 4, cudaMemcpyHostToDevice, s->stream));
     WK_CUDA_CHECK(cudaMemcpyAsync(s->pos_dev, zeros.data(), B * 4, cudaMemcpyHostToDevice, s->stream));
-    WK_CHECK(decoder_forward(s, 0, s->pos_dev, use_fused(s)));
+    WK_CHECK(decoder_forward(s, 0, 0, s->pos_dev, use_fused(s)));
     // currentTokens = [SOT] for every window: reuse the decode-state arrays as the stateless token history
     WK_CUDA_CHECK(cudaMemcpyAsync(s->st.tokens, ids.data(), B * 4, cudaMemcpyHostToDevice, s->stream));   // ld_tokens = 1
     WK_CUDA_CHECK(cudaMemcpyAsync(s->st.n_tokens, ones.data(), B * 4, cudaMemcpyHostToDevice, s->stream));
@@ -1066,6 +1131,22 @@ wk_status wk_transcribe_windows(wk_model* m, wk_session* s, const float* pcm_hos
 wk_status wk_session_stats(const wk_session* s, int64_t* out4) {
     if (!s || !out4) return WK_ERR_INVALID_ARGUMENT;
     memcpy(out4, s->stats, sizeof(s->stats));
+    return WK_OK;
+}
+
+wk_status wk_session_set_language_tokens(wk_session* s, const int32_t* tokens, int32_t n) {
+    if (!s || n < 0 || n > 4096 || (n > 0 && !tokens)) { set_error("wk_session_set_language_tokens: bad arguments (n %d, limit 4096)", n); return WK_ERR_INVALID_ARGUMENT; }
+    for (int i = 0; i < n; ++i)
+        if (tokens[i] < 0 || tokens[i] >= s->m->cfg.vocab) { set_error("wk_session_set_language_tokens: token %d outside the vocabulary", tokens[i]); return WK_ERR_INVALID_ARGUMENT; }
+    s->lang_list.assign(tokens, tokens + n);
+    return WK_OK;
+}
+
+wk_status wk_session_languages(const wk_session* s, int64_t n, int32_t* tokens, float* logprobs) {
+    if (!s || n < 0 || (n > 0 && !tokens)) { set_error("wk_session_languages: bad arguments"); return WK_ERR_INVALID_ARGUMENT; }
+    if (n > (int64_t)s->win_lang_tok.size()) { set_error("wk_session_languages: %lld windows asked, the last call had %zu", (long long)n, s->win_lang_tok.size()); return WK_ERR_INVALID_ARGUMENT; }
+    if (n > 0) memcpy(tokens, s->win_lang_tok.data(), (size_t)n * 4);
+    if (n > 0 && logprobs) memcpy(logprobs, s->win_lang_lp.data(), (size_t)n * 4);
     return WK_OK;
 }
 

@@ -618,6 +618,22 @@ int32_t wk_tokenizer_split_to_word_tokens(const wk_tokenizer* t, const int32_t* 
     return (int32_t)words.size();
 }
 
+int32_t wk_tokenizer_language_tokens(const wk_tokenizer* t, int32_t* out, int32_t cap) {
+    if (!t || cap < 0 || (cap > 0 && !out)) return -1;
+    std::vector<int32_t> ids;   // "<|xx|>" / "<|xxx|>": the language codes among the added tokens
+    for (size_t id = 0; id < t->id_to_token.size(); ++id) {
+        if (!t->present[id] || !t->added[id]) continue;
+        const std::string& s = t->id_to_token[id];
+        if (s.size() < 6 || s.size() > 7 || s.compare(0, 2, "<|") != 0 || s.compare(s.size() - 2, 2, "|>") != 0) continue;
+        bool letters = true;
+        for (size_t i = 2; i + 2 < s.size(); ++i) letters &= s[i] >= 'a' && s[i] <= 'z';
+        if (letters) ids.push_back((int32_t)id);
+    }
+    if ((int64_t)ids.size() > cap) return -(int32_t)ids.size();   // -(ids needed)
+    if (!ids.empty()) memcpy(out, ids.data(), ids.size() * 4);
+    return (int32_t)ids.size();
+}
+
 static int32_t hook_split(void* user, const int32_t* tokens, int32_t n, char* text, int32_t text_cap, int32_t* counts, int32_t counts_cap) {
     return wk_tokenizer_split_to_word_tokens((const wk_tokenizer*)user, tokens, n, text, text_cap, counts, counts_cap);
 }

@@ -141,9 +141,10 @@ class VADAudioChunker:
 
 def transcribe_streams(kit, audioArrays: Sequence[np.ndarray], options: Optional[DecodingOptions] = None,
                        clipTimestamps: Sequence[float] = (), windowClipTime: float = 1.0, maxWindowSeek: Optional[int] = None,
-                       chunkingStrategy: Optional[str] = None, split_to_word_tokens=None, decode=None, hooks=None):
+                       chunkingStrategy: Optional[str] = None, split_to_word_tokens=None, decode=None, hooks=None, languages: Optional[list] = None):
     """TranscribeTask.run's seek loop for many audio arrays at once (TranscribeTask.swift:98-279; `chunkingStrategy="vad"`
-    = WhisperKit.swift:878-911).  Returns (segments per stream, number of 30 s windows decoded)."""
+    = WhisperKit.swift:878-911).  Returns (segments per stream, number of 30 s windows decoded).  A `languages` list receives each
+    stream's TranscriptionResult.language as (token, log-probability) (wk_transcription_language)."""
     opts = kit.resolveLanguage(options or DecodingOptions())   # DecodingOptions.language -> <|xx|> through the tokenizer
     lib = kit.model.lib
     arrs = [np.ascontiguousarray(a, dtype=np.float32) for a in audioArrays]
@@ -181,6 +182,11 @@ def transcribe_streams(kit, audioArrays: Sequence[np.ndarray], options: Optional
                 segs[w.segment].words.append(WordTiming(w.word.decode("utf-8"), [int(w.tokens[k]) for k in range(w.n_tokens)], float(w.start),
                                                         float(w.end), float(w.probability), int(w.segment)))
         windows = lib.wk_transcription_window_count(h)
+        if languages is not None:
+            tok, lp = C.c_int32(), C.c_float()
+            for i in range(len(arrs)):
+                check(lib.wk_transcription_language(h, i, C.byref(tok), C.byref(lp)))
+                languages.append((int(tok.value), float(lp.value)))
     finally:
         lib.wk_transcription_free(h)
     per_stream = [[g for g in segs if g.stream == i] for i in range(len(arrs))]
@@ -193,6 +199,9 @@ class TranscriptionResult:
     text: str
     segments: List[TranscriptionSegment]
     windows: int = 0
+    languageToken: Optional[int] = None
+    languageLogProb: float = 0.0
+    language: Optional[str] = None      # the code, with a tokenizer
 
 
 def transcribe_audio(kit, audioArrays: Sequence[np.ndarray], options: Optional[DecodingOptions] = None, tokenizer=None,
@@ -206,15 +215,18 @@ def transcribe_audio(kit, audioArrays: Sequence[np.ndarray], options: Optional[D
         raise _lib.WhisperError(-1, "wordTimestamps needs a tokenizer")
     native = tokenizer.hooks() if (tokenizer is not None and opts.wordTimestamps and hasattr(tokenizer, "hooks")) else None
     split = tokenizer.splitToWordTokens if (tokenizer is not None and opts.wordTimestamps and native is None) else None
+    langs = []
     per_stream, windows = transcribe_streams(kit, audioArrays, opts, clipTimestamps=clipTimestamps, chunkingStrategy=chunkingStrategy,
-                                             split_to_word_tokens=split, decode=tokenizer.decode if split is not None else None, hooks=native)
+                                             split_to_word_tokens=split, decode=tokenizer.decode if split is not None else None, hooks=native,
+                                             languages=langs)
     sb = kit.specialTokens.specialTokenBegin
     out = []
-    for segs in per_stream:
+    for segs, (ltok, llp) in zip(per_stream, langs):
         text = ""
         if tokenizer is not None:
             for g in segs:
                 g.text = tokenizer.decode([t for t in g.tokens if t < sb] if opts.skipSpecialTokens else g.tokens)
             text = tokenizer.decode([t for g in segs for t in g.tokens if t < sb]).strip(" \t               　")
-        out.append(TranscriptionResult(text, segs, windows))
+        code = tokenizer.decode([ltok]).removeprefix("<|").removesuffix("|>") if tokenizer is not None else None
+        out.append(TranscriptionResult(text, segs, windows, ltok, llp, code))
     return out

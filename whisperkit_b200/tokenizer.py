@@ -69,6 +69,18 @@ class WhisperTokenizer:
                              timeTokenBegin=st.time_token_begin, transcribeToken=st.transcribe_token, translateToken=st.translate_token,
                              whitespaceToken=st.whitespace_token)
 
+    @property
+    def allLanguageTokens(self) -> List[int]:
+        """WhisperTokenizerWrapper.allLanguageTokens (Models.swift:1219): the "<|xx|>" / "<|xxx|>" ids of the vocabulary, ascending."""
+        n = self.lib.wk_tokenizer_language_tokens(self.handle, None, 0)
+        if n == 0:
+            return []
+        arr = (C.c_int32 * -n)()
+        n = self.lib.wk_tokenizer_language_tokens(self.handle, arr, -n)
+        if n < 0:
+            raise _lib.WhisperError(-1, "wk_tokenizer_language_tokens failed")
+        return [int(v) for v in arr[:n]]
+
     def splitToWordTokens(self, tokenIds: Sequence[int]) -> Tuple[List[str], List[List[int]]]:
         n = len(tokenIds)
         arr = (C.c_int32 * max(1, n))(*[int(t) for t in tokenIds])
